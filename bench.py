@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200 Newton iteration core.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--N 100]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--N 100] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], the configuration the metric is quoted on): 3D Brusselator N=100 (10^6 cells, 2*10^6
 unknowns), NewtonRaphson(linsolve = KrylovJL_GMRES()) with the matrix-free exact JVP, abstol = 1e-8 (the reference
@@ -25,6 +25,8 @@ BASELINE configuration, each with its own CPU baseline (rank 0 only, after the t
   `precond`    config 3 with the multigrid `precs` + EisenstatWalkerForcing2 (Arnoldi iterations, Newton steps/s);
   `ensemble`   config 5: 8192 x (2D N=32), sharded over the ranks, gathered through the library's C-ABI collective.
 `--impl reference` times the CPU restatement of the reference (oracle/, "port": the Julia reference cannot run here).
+`--dump-outputs DIR` writes what the last timed headline step returned (see `dump_outputs`), so that two builds can be compared
+output for output on the same deterministic inputs.
 """
 import argparse
 import json
@@ -451,6 +453,30 @@ def leg_precond(nls, torch, ctx):
     return out
 
 
+DUMP_LIMIT = 64 * 10 ** 6  # bytes, all files of --dump-outputs together
+
+
+def dump_outputs(out_dir, sol, trace_fields):
+    """What a caller of the timed path receives from its last step, as float64 arrays in out_dir/<name>.npy:
+      u, resid      the root and the residual there (length n; when both no longer fit DUMP_LIMIT, the same seeded sample of
+                    their entries, whose indices go to sample_index.npy);
+      stats         retcode, nsteps, nf, njacs, nfactors, nsolve, njvp, resid_inf;
+      trace         one row per Newton iteration, one column per trace field in `trace_fields` order."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    s = sol.stats
+    out = {"u": sol.u.to_host(), "resid": sol.resid.to_host(),
+           "stats": [sol.retcode, s.nsteps, s.nf, s.njacs, s.nfactors, s.nsolve, s.njvp, sol.resid_inf],
+           "trace": np.array([[getattr(t, k) for k in trace_fields] for t in sol.trace], dtype=np.float64).reshape(-1, len(trace_fields))}
+    n = out["u"].size
+    keep = (DUMP_LIMIT - 10 ** 6) // (3 * 8)  # u, resid and the sample index; 1 MB left for stats and trace
+    if n > keep:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        out["u"], out["resid"], out["sample_index"] = out["u"][idx], out["resid"][idx], idx
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def traffic_from_profile(bytes_per_launch, resident):
     p = os.path.join(ROOT, "profiles", "r2_resident_traffic.json")
     if resident and os.path.exists(p):
@@ -528,6 +554,8 @@ def run_b200(args):
     ctx.profile(False, reset=False)
     clk = clocks.stop() if rank == 0 else None
     assert sol.retcode == nls.ReturnCode.Success and sol.resid_inf < 1e-8, (sol.retcode, sol.resid_inf)
+    if args.dump_outputs and rank == 0:  # before the e2e region reuses the cache's buffers that sol.u and sol.resid point into
+        dump_outputs(args.dump_outputs, sol, [k for k, _ in nls.abi.TraceRec._fields_])
     # ---- end-to-end timed region: host buffers, H2D + D2H inside
     barrier()
     e2, e3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -652,7 +680,12 @@ def main():
     ap.add_argument("--orth", default="mgs", choices=["mgs", "cgs2"], help="GMRES orthogonalisation: mgs = Krylov.jl default (reference), cgs2 = reorthogonalised")
     ap.add_argument("--no-ensemble", dest="no_ensemble", action="store_true", help="skip the config-5 ensemble leg")
     ap.add_argument("--no-legs", dest="no_legs", action="store_true", help="skip the n80 / lu / sparse_tr / precond legs (configs 2, 4 and the §8f variants)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", help="write the last timed step's outputs (u, resid, stats, trace) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200: the reference arm times a sample of the solve, not the whole path")
     with _OneLineStdout() as out:
         _OUT = out
         if args.impl == "reference":
